@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA probe
     python bench.py --impl reference --gpus N --steps K ...   # the reference's CPU/NVML poll
     python bench.py --config c2|c3-full|c5 ...                # BASELINE configs 2 / 3 (full mode) / 5 (storm)
+    python bench.py ... --dump-outputs DIR                    # also write the last timed step's results as DIR/*.npy
 
 A "step" is one pass of the hot path: one `cdprobe_run` over the N-GPU domain (sliced mode,
 1 GiB per GPU, read + write + verify) — BASELINE.json configs[2] at N GPUs; at N = 1 the same
@@ -34,6 +35,8 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+# the benchmark leaves the tree as the build left it (it may be read-only): no bytecode caches next to the sources
+sys.dont_write_bytecode = True
 
 GIB = 1 << 30
 NVLINK_PEAK_GBPS = 900.0        # nominal per direction per GPU (BASELINE.md §2)
@@ -169,7 +172,7 @@ def cpu_poll_timing(n_gpus: int, steps: int, warmup: int, budget_s: float, flags
     per GPU."""
     from oracle import oracle as o
 
-    o.build()
+    o.lib()
     times, last = [], None
     t_stop = time.perf_counter() + budget_s
     for i in range(warmup + steps):
@@ -279,6 +282,25 @@ def parity_block(pkg, oracle, res, n, nbytes, mode_id, uuids, seed):
         block["reach_vs_nvml_ok"] = None
         block["reach_vs_nvml_error"] = str(e)
     return block
+
+
+def dump_outputs(res, out_dir):
+    """Writes the N x N matrices the last timed cdprobe_run handed its caller (completed across ranks) as
+    out_dir/<name>.npy, so that two builds run with the same arguments can be compared file for file.
+    Every value written is computed, not measured: the source patterns are seeded and the write pattern is
+    salted by the run count, which the arguments fix.  The per-pair GB/s and the timings differ from run to
+    run and stay in the JSON line.  A 64-bit checksum does not fit a float64 mantissa, so each one is stored
+    as its (high, low) 32-bit halves along a last axis of length 2."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"reach_read": np.array(res.reach_read, np.float32), "reach_write": np.array(res.reach_write, np.float32),
+              "status": np.array(res.status, np.float32)}
+    for name in ("sum_read", "xor_read", "sum_write", "xor_write"):
+        a = np.array(getattr(res, name), np.uint64)
+        arrays[name] = np.stack([a >> np.uint64(32), a & np.uint64(0xFFFFFFFF)], axis=-1).astype(np.float64)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def run_probe(args):
@@ -413,8 +435,10 @@ def run_probe(args):
     if rank == 0:
         from oracle import oracle as o  # the checker: never on the measured path
 
-        o.build()
+        o.lib()
         parity = parity_block(pkg, o, res, n, args.bytes, mode_id, uuids, o.DEFAULT_SEED)
+        if args.dump_outputs:
+            dump_outputs(res, args.dump_outputs)
     parity_ok = grp.gather_objects(None if parity is None else
                                    bool(parity["checksum_ok"] and parity["reach_vs_nvml_ok"] is not False))[0]
 
@@ -717,8 +741,10 @@ def run_storm(args, pkg, probe, grp, info, n, rank, local, daemon_cost, conf):
     if rank == 0:
         from oracle import oracle as o
 
-        o.build()
+        o.lib()
         parity = parity_block(pkg, o, res, n, args.bytes, 1, uuids, o.DEFAULT_SEED)
+        if args.dump_outputs:
+            dump_outputs(res, args.dump_outputs)
         line = {"metric": "nvlink_probe_ms", "value": stats["probe_ms_p50"], "unit": "ms", "n_gpus": n, "steps": cycles,
                 "warmup": max(args.warmup, 3), "ms_per_step": stats["wall_ms"] / cycles, "higher_is_better": False,
                 "scaling": "weak", "vs_baseline": None, "dtype": "u64", "data": "synthetic",
@@ -755,7 +781,14 @@ def main():
                     help="BASELINE.json configs beyond the headline: c2 (2 GPUs, 64 MiB, full), c3-full (1 GiB per ordered "
                          "pair), c5 (reconcile storm: --steps cycles)")
     ap.add_argument("--all-rank-barriers", action="store_true", help="round-1 barrier schedule (comparison)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write the reachability, status and checksum matrices of the last "
+                         "timed step as DIR/<name>.npy (rank 0; the same arguments give the same files)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the probe's results; the reference arm has none")
     if args.impl == "reference":
         return run_reference(args)
     return run_probe(args)

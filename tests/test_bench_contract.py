@@ -195,3 +195,61 @@ def test_bench_runs_end_to_end_with_parity(tmp_path):
     j = json.loads(lines[0])
     assert j["n_gpus"] == 1 and j["gpu_launches"] == 10 and j["parity"]["checksum_ok"] is True
     assert j["parity"]["reach_vs_nvml_ok"] is True and j["verdict"] is True and 0.5 < j["roofline"]["frac"] < 1.1
+
+
+def _load_dump(d):
+    import numpy as np
+
+    out = {}
+    for f in sorted(os.listdir(d)):
+        a = np.load(os.path.join(d, f))
+        assert a.dtype in (np.float32, np.float64), (f, a.dtype)
+        out[f[:-len(".npy")]] = a
+    return out
+
+
+def test_dump_outputs_keeps_every_checksum_bit(tmp_path):
+    """--dump-outputs stores float arrays only: a u64 checksum goes out as its exact (high, low) 32-bit halves."""
+    import types
+
+    import numpy as np
+
+    import bench
+
+    n = 2
+    big = [[0xFFFFFFFFFFFFFFFF, 0x8000000000000001], [(1 << 53) + 1, 12345]]
+    r = types.SimpleNamespace(reach_read=[[1, 0], [1, 1]], reach_write=[[1, 1], [0, 1]], status=[[0, -4], [0, 0]],
+                              sum_read=big, xor_read=big, sum_write=big, xor_write=big)
+    bench.dump_outputs(r, str(tmp_path / "out"))
+    d = _load_dump(tmp_path / "out")
+    assert set(d) == {"reach_read", "reach_write", "status", "sum_read", "xor_read", "sum_write", "xor_write"}
+    assert d["reach_read"].tolist() == r.reach_read and d["status"].tolist() == r.status
+    for name in ("sum_read", "xor_read", "sum_write", "xor_write"):
+        a = d[name]
+        assert a.shape == (n, n, 2)
+        assert [[(int(a[i, j, 0]) << 32) | int(a[i, j, 1]) for j in range(n)] for i in range(n)] == big
+
+
+@pytest.mark.gpu
+def test_bench_dump_outputs_repeat_and_match_the_oracle(tmp_path, oracle):
+    """Two runs with the same arguments dump the same files; the dumped read checksum is the oracle's, and the
+    dumped matrices are the ones the line's parity block checked."""
+    import subprocess
+    import sys
+
+    nbytes = 16 << 20
+    dumps = []
+    for k in range(2):
+        d = tmp_path / f"out{k}"
+        cp = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--gpus", "1", "--steps", "5", "--warmup", "3",
+                             "--bytes", str(nbytes), "--no-cpu-baseline", "--no-daemon", "--dump-outputs", str(d)],
+                            capture_output=True, text=True, timeout=300)
+        assert cp.returncode == 0, cp.stderr[-2000:]
+        j = json.loads([l for l in cp.stdout.splitlines() if l.startswith("{")][-1])
+        assert j["steps"] == 5 and j["parity"]["checksum_ok"] is True
+        dumps.append(_load_dump(d))
+    a, b = dumps
+    assert set(a) == set(b) and all((a[k] == b[k]).all() for k in a)
+    assert a["reach_read"].tolist() == a["reach_write"].tolist() == [[1.0]] and a["status"].tolist() == [[0.0]]
+    s, x = (int(a[k][0, 0, 0]) << 32 | int(a[k][0, 0, 1]) for k in ("sum_read", "xor_read"))
+    assert (s, x) == oracle.expected_read(oracle.DEFAULT_SEED, 1, nbytes, 1, 0, 0, True)
