@@ -262,7 +262,7 @@ CDPROBE_API const char* cdprobe_last_error(void);
  *   cdprobe_strerror / cdprobe_last_error   text of the Go error:   fmt.Errorf convention of main.go
  *   cdprobe_remap_peer / cdprobe_unmap_peer  emulate NodeUnprepare/NodePrepare churn around a live domain:
  *                                                                   cmd/compute-domain-kubelet-plugin/driver.go:165-232
- *   cdprobe_gather, cdprobe_info, cdprobe_trace, cdprobe_set_option, cdprobe_corrupt, cdprobe_plan,
+ *   cdprobe_gather, cdprobe_info, cdprobe_trace, cdprobe_set_option, cdprobe_corrupt, cdprobe_peek, cdprobe_plan,
  *   cdprobe_schedule, cdprobe_gate, cdprobe_ce_copy, cdprobe_rendezvous_selftest: diagnostics, benches, fault injection; the reference has
  *   no counterpart (it has no probe, SURVEY.md F1).
  */
@@ -303,8 +303,12 @@ CDPROBE_API int cdprobe_ce_copy(cdprobe_t* h, uint32_t n_copies, const uint32_t*
 CDPROBE_API int cdprobe_remap_peer(cdprobe_t* h, uint32_t local, uint32_t peer);
 /* Fault injection for parity tests: drop local rank's mapping of `peer` (cell becomes unreachable, run still returns). */
 CDPROBE_API int cdprobe_unmap_peer(cdprobe_t* h, uint32_t local, uint32_t peer);
-/* Fault injection: XOR one 64-bit word of local rank's source slice / force a bad write salt. */
+/* Fault injection: XOR one 64-bit word of local rank's source buffer (`byte_offset` from the start of the source). */
 CDPROBE_API int cdprobe_corrupt(cdprobe_t* h, uint32_t local, uint64_t byte_offset, uint64_t xor_mask);
+/* Diagnostics: copy `bytes` from local rank `local`'s own probe allocation, starting `byte_offset` bytes from its
+ * base (Ctrl at 0, source at 2 MiB, landing slots after the source rounded up to 2 MiB; DESIGN §4), into `out`.
+ * Ordered after everything enqueued on that rank's stream (a finished cdprobe_run). Never reads outside the allocation. */
+CDPROBE_API int cdprobe_peek(cdprobe_t* h, uint32_t local, uint64_t byte_offset, uint64_t bytes, void* out);
 CDPROBE_API void cdprobe_close(cdprobe_t* h);
 
 /* Host-only helpers (no CUDA): schedule + slice arithmetic; the fd/blob rendezvous self-test. */

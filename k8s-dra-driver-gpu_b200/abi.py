@@ -199,6 +199,7 @@ SYMBOLS = {
     "cdprobe_remap_peer": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32]),
     "cdprobe_unmap_peer": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32]),
     "cdprobe_corrupt": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint64, C.c_uint64]),
+    "cdprobe_peek": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint64, C.c_uint64, C.c_void_p]),
     "cdprobe_ce_copy": (C.c_int, [C.c_void_p, C.c_uint32, C.POINTER(C.c_uint32), C.POINTER(C.c_uint32), C.c_uint32,
                                   C.c_uint64, C.c_uint32, C.POINTER(C.c_double)]),
     "cdprobe_close": (None, [C.c_void_p]),

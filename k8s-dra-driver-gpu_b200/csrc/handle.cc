@@ -1133,6 +1133,19 @@ int cdprobe_corrupt(cdprobe_t* h, uint32_t local, uint64_t byte_offset, uint64_t
   return CDPROBE_OK;
 }
 
+int cdprobe_peek(cdprobe_t* h, uint32_t local, uint64_t byte_offset, uint64_t bytes, void* out) {
+  if (h == nullptr || out == nullptr || local >= h->n_local || bytes == 0) return CDPROBE_ERR_ARG;
+  const uint64_t alloc = h->plan.alloc_bytes;
+  if (byte_offset > alloc || bytes > alloc - byte_offset) return CDPROBE_ERR_ARG;  // no overflow in offset + bytes
+  if (h->sticky) return CDPROBE_ERR_STATE;
+  cdp::LocalRank& L = h->lr[local];
+  CDP_RT(cudaSetDevice(L.ordinal));
+  const uint8_t* p = reinterpret_cast<const uint8_t*>(L.va[L.grank]) + byte_offset;
+  CDP_RT(cudaMemcpyAsync(out, p, bytes, cudaMemcpyDeviceToHost, L.stream));
+  CDP_RT(cudaStreamSynchronize(L.stream));
+  return CDPROBE_OK;
+}
+
 int cdprobe_ce_copy(cdprobe_t* h, uint32_t n_copies, const uint32_t* local, const uint32_t* peer, uint32_t push,
                     uint64_t bytes, uint32_t reps, double* ms_out) {
   cdp::g_last_error.clear();

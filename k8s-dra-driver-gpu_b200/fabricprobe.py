@@ -244,6 +244,14 @@ class Probe:
         if rc != abi.OK:
             _raise(self._lib, rc, "cdprobe_corrupt")
 
+    def Peek(self, local: int, byte_offset: int, nbytes: int) -> bytes:
+        """`nbytes` of local rank `local`'s own allocation from `byte_offset` (Ctrl, source, landing slots; DESIGN §4)."""
+        buf = C.create_string_buffer(nbytes) if nbytes > 0 else None
+        rc = self._lib.cdprobe_peek(self._h, local, byte_offset, nbytes, buf)
+        if rc != abi.OK:
+            _raise(self._lib, rc, "cdprobe_peek")
+        return buf.raw
+
     def Close(self) -> None:
         if self._h:
             self._lib.cdprobe_close(self._h)

@@ -150,6 +150,46 @@ def write_checksum(seed: int, src: int, dst: int, run_seq: int, n_words: int):
     return s.value, x.value
 
 
+_GOLDEN = 0x9E3779B97F4A7C15
+_WRITE_TAG = 0x5752495445  # "WRITE"
+_M64 = (1 << 64) - 1
+
+
+def _splitmix64_np(x):
+    """pattern.c's cdoracle_splitmix64 over a numpy.uint64 array (wrapping arithmetic)."""
+    import numpy as np
+
+    u = np.uint64
+    z = x + u(_GOLDEN)
+    z ^= z >> u(30)
+    z *= u(0xBF58476D1CE4E5B9)
+    z ^= z >> u(27)
+    z *= u(0x94D049BB133111EB)
+    z ^= z >> u(31)
+    return z
+
+
+def src_words(seed: int, rank: int, first_word: int, n: int):
+    """Words first_word .. first_word + n - 1 of rank `rank`'s source buffer, as a numpy.uint64 array
+    (vectorised restatement of cdoracle_src_word: splitmix64(seed ^ rank << 56 ^ k))."""
+    import numpy as np
+
+    k = np.arange(n, dtype=np.uint64) + np.uint64(first_word)
+    return _splitmix64_np(k ^ np.uint64((seed ^ (rank << 56)) & _M64))
+
+
+def write_words(seed: int, src: int, dst: int, run_seq: int, first_word: int, n: int):
+    """Words first_word .. first_word + n - 1 of what rank `src` stores into rank `dst`'s landing slot in run
+    `run_seq`, as a numpy.uint64 array (cdoracle_write_salt + cdoracle_write_word: z = (salt + k) * golden,
+    w = z ^ z >> 32)."""
+    import numpy as np
+
+    x = (seed ^ _WRITE_TAG ^ (src << 56) ^ (dst << 48) ^ run_seq) & _M64
+    salt = _splitmix64_np(np.array([x], dtype=np.uint64))[0]
+    z = (np.arange(n, dtype=np.uint64) + np.uint64(first_word) + salt) * np.uint64(_GOLDEN)
+    return z ^ (z >> np.uint64(32))
+
+
 def plan(n: int, nbytes: int, mode: int, diag: bool = False) -> PlanT:
     p = PlanT()
     rc = lib().cdoracle_plan(n, nbytes, mode, 1 if diag else 0, C.byref(p))

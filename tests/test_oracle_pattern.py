@@ -46,7 +46,7 @@ def test_buffer_checksum_equals_streaming(oracle):
 
 
 def test_checksum_is_position_sensitive_across_granules(oracle):
-    # swapping two 16 KiB granules keeps S but changes X (a misplaced chunk is detected)
+    # swapping granules 0 and 1 (fold6 0 and 1) keeps S but changes X; equal fold6 is a blind spot, pinned below
     L = oracle.lib()
     n = 2048 * 3
     words = (C.c_uint64 * n)()
@@ -59,6 +59,82 @@ def test_checksum_is_position_sensitive_across_granules(oracle):
     s1, x1 = C.c_uint64(), C.c_uint64()
     L.cdoracle_checksum(words, n, C.byref(s1), C.byref(x1))
     assert s0.value == s1.value and x0.value != x1.value
+
+
+def test_numpy_pattern_equals_c_oracle_and_golden(oracle, golden):
+    """src_words / write_words (the reference the read-back tests compare HBM with) word for word against the
+    scalar C oracle: golden vectors, random words, and k near 2^29, 2^32 and 2^40 (byte offsets past 4 GiB)."""
+    import random
+
+    L = oracle.lib()
+    for v in golden["src_words"]:
+        assert int(oracle.src_words(int(v["seed"]), v["rank"], v["k"], 1)[0]) == int(v["word"])
+    for v in golden["write_words"]:
+        got = oracle.write_words(int(v["seed"]), v["src"], v["dst"], v["run_seq"], v["k"], 1)
+        assert int(got[0]) == int(v["word"])
+    rng = random.Random(7)
+    starts = [0, 1, 2047, (1 << 29) - 5, 1 << 29, (1 << 32) - 5, 1 << 32, (1 << 40) - 5, (1 << 40) + 3]
+    starts += [rng.getrandbits(64) >> rng.randrange(0, 40) for _ in range(20)]
+    for k0 in starts:
+        seed, rank, dst, run_seq = rng.getrandbits(64), rng.randrange(16), rng.randrange(16), rng.getrandbits(32)
+        n = 9
+        k0 = min(k0, (1 << 64) - n)
+        src = oracle.src_words(seed, rank, k0, n)
+        assert [int(w) for w in src] == [L.cdoracle_src_word(seed, rank, k0 + i) for i in range(n)], hex(k0)
+        salt = L.cdoracle_write_salt(seed, rank, dst, run_seq)
+        wr = oracle.write_words(seed, rank, dst, run_seq, k0, n)
+        assert [int(w) for w in wr] == [L.cdoracle_write_word(salt, k0 + i) for i in range(n)], hex(k0)
+    # a long run agrees with the oracle's streamed checksum too
+    words = oracle.src_words(oracle.DEFAULT_SEED, 3, 5000, 2048 * 5 + 17)
+    assert _checksum(oracle, words) == oracle.src_checksum(oracle.DEFAULT_SEED, 3, 5000, len(words))
+
+
+def _checksum(oracle, words):
+    s, x = C.c_uint64(), C.c_uint64()
+    oracle.lib().cdoracle_checksum(words.ctypes.data_as(C.POINTER(C.c_uint64)), len(words), C.byref(s), C.byref(x))
+    return s.value, x.value
+
+
+def test_checksum_blind_spots_are_pinned(oracle):
+    """What the (S, X) checksum cannot see (DESIGN §5).  These mutations of a 70-granule source leave S and X
+    unchanged; the read-back tests (tests/test_gpu_readback.py), not the checksum, guard kernel placement.  If
+    the checksum is strengthened, this test fails and should be turned around knowingly."""
+    import numpy as np
+
+    G, U = 2048, 1024  # words per 16 KiB granule / per 8 KiB unit
+    base = oracle.src_words(oracle.DEFAULT_SEED, 0, 0, 70 * G)
+    ref = _checksum(oracle, base)
+
+    def mutated(fn):
+        w = base.copy()
+        fn(w)
+        return _checksum(oracle, w)
+
+    def swap_words(w):  # two words of granule 2
+        w[2 * G + 5], w[2 * G + 700] = w[2 * G + 700], w[2 * G + 5]
+
+    def swap_units(w):  # the two 8 KiB units (TMA stages / warp work units) of granule 4
+        w[4 * G:4 * G + U], w[4 * G + U:5 * G] = w[4 * G + U:5 * G].copy(), w[4 * G:4 * G + U].copy()
+
+    def balanced_bit_flips(w):  # bit 9 goes 0 -> 1 in one word and 1 -> 0 in another word of granule 6
+        bit = 1 << 9
+        lo = next(k for k in range(6 * G, 7 * G) if not int(w[k]) & bit)
+        hi = next(k for k in range(6 * G, 7 * G) if int(w[k]) & bit)
+        w[lo] ^= np.uint64(bit)
+        w[hi] ^= np.uint64(bit)
+
+    def swap_granules(a, b):
+        def fn(w):
+            w[a * G:(a + 1) * G], w[b * G:(b + 1) * G] = w[b * G:(b + 1) * G].copy(), w[a * G:(a + 1) * G].copy()
+        return fn
+
+    assert mutated(swap_words) == ref
+    assert mutated(swap_units) == ref
+    assert mutated(balanced_bit_flips) == ref
+    assert mutated(swap_granules(0, 65)) == ref  # fold6(0) == fold6(65) == 0
+    assert mutated(swap_granules(1, 64)) == ref  # fold6(1) == fold6(64) == 1
+    s, x = mutated(swap_granules(3, 5))
+    assert s == ref[0] and x != ref[1]  # different fold6: detected
 
 
 def test_plans_match_golden(oracle, golden):
