@@ -291,6 +291,17 @@ CDPROBE_API int cdprobe_trace(cdprobe_t* h, uint32_t local, cdprobe_trace_t* out
                                         self-contained kernel is what `ncu` can replay: NVLink byte counters per launch. */
 #define CDPROBE_OPT_ALL_RANK_BARRIERS 15u /* value 0/1: see CDPROBE_FLAG_ALL_RANK_BARRIERS */
 #define CDPROBE_OPT_PAIR_BARRIERS 16u     /* value 0/1: see CDPROBE_FLAG_PAIR_BARRIERS */
+#define CDPROBE_OPT_DEBUG_DAMAGE_WRITE 17u /* fault injection: value = ((local rank + 1) << 16) | (target rank << 8) | code,
+                                              0 = off.  In every run while set, once that local rank's write job into
+                                              `target`'s landing slot is over and before anyone is told so, the kernel
+                                              damages the slot (the writer's own checksum stays that of the clean
+                                              pattern): 1 = flip bit 0 of the first word (S and X change); 2 = flip
+                                              bit 63 of the last word; 3 = add 0x9E3779B97F4A7C15 to the first word
+                                              and subtract it from the last (S unchanged, only X sees it); 4 = swap words
+                                              0 and 1 (S and X unchanged: a blind spot of the checksum, the verify
+                                              passes).  ERR_ARG for a bad local rank, a target past the domain or
+                                              the rank itself when the diagonal is not probed, or a code outside
+                                              1..4. */
 CDPROBE_API int cdprobe_set_option(cdprobe_t* h, uint32_t option, uint64_t value);
 /* Copy-engine reference on the probe's own buffers (the same-box ceiling the roofline is quoted against; not part
  * of a probe): copy k moves `bytes` (capped at the source / landing size) `reps` times back to back between local

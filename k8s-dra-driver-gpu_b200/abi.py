@@ -32,6 +32,7 @@ OPT_UNIDIRECTIONAL = 7
 OPT_WARMUP, OPT_WARMUP_BYTES, OPT_DEBUG_SKIP_RANK = 8, 9, 10
 OPT_CTAS_RANK, OPT_MIN_FRACTION_PPM, OPT_LINK_PEAK_MBPS, OPT_SOLO_RANK, OPT_ALL_RANK_BARRIERS = 11, 12, 13, 14, 15
 OPT_PAIR_BARRIERS = 16
+OPT_DEBUG_DAMAGE_WRITE = 17
 
 _N2 = MAX_GPUS * MAX_GPUS
 

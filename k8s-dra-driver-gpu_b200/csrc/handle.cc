@@ -99,6 +99,7 @@ struct cdprobe {
   bool warm_now = false;
   uint32_t debug_skip_rank = 0;  // 1-based local rank whose kernel is NOT launched (fault injection)
   uint32_t solo_rank = 0;        // 1-based local rank that runs alone, no cross-GPU barrier (ncu captures)
+  uint32_t damage_write = 0;     // CDPROBE_OPT_DEBUG_DAMAGE_WRITE value (fault injection; 0 = off)
   double last_probe_ms = 0.0;    // host wall clock of the previous run (wait_rows: how long to spin hot)
   uint32_t verify_ctas = 32;  // CTAs that verify landing slots under CDPROBE_FLAG_OVERLAP_VERIFY
   double open_ms = 0, fill_ms = 0;
@@ -239,6 +240,10 @@ static void fill_params(const cdprobe* h, uint32_t li, const Phase* phases, uint
     for (int jb = 0; jb < 2; ++jb) {
       Job& job = P->phase[p].job[jb];
       if (job.kind == kJobWrite) job.salt = write_salt(h->seed, L.grank, (uint32_t)job.peer, h->launch_seq);
+      // fault injection: the writer byte is unused on write jobs; nonzero = damage code the barrier applies
+      if (job.kind == kJobWrite && h->damage_write != 0 && (h->damage_write >> 16) == li + 1 &&
+          ((h->damage_write >> 8) & 0xffu) == (uint32_t)job.peer)
+        job.writer = (uint8_t)(h->damage_write & 0xffu);
       if (job.kind == kJobWarm) job.salt = h->warm_now ? h->warm_bytes : 0ull;
     }
   }
@@ -1079,6 +1084,18 @@ int cdprobe_set_option(cdprobe_t* h, uint32_t option, uint64_t value) {
     case CDPROBE_OPT_WARMUP_BYTES:
       h->warm_bytes = value / 128 * 128;
       return CDPROBE_OK;
+    case CDPROBE_OPT_DEBUG_DAMAGE_WRITE:
+    {
+      if (value == 0) {
+        h->damage_write = 0;
+        return CDPROBE_OK;
+      }
+      const uint64_t li = value >> 16, target = (value >> 8) & 0xffu, code = value & 0xffu;
+      if (li == 0 || li > h->n_local || target >= h->n_total || code < 1 || code > 4) return CDPROBE_ERR_ARG;
+      if (target == h->lr[li - 1].grank && !h->plan.diag) return CDPROBE_ERR_ARG;  // no write job into itself
+      h->damage_write = (uint32_t)value;
+      return CDPROBE_OK;
+    }
     case CDPROBE_OPT_VERIFY_CTAS:
       if (value == 0 || value > 65535) return CDPROBE_ERR_ARG;
       h->verify_ctas = (uint32_t)value;

@@ -486,6 +486,36 @@ __device__ void publish_verdicts(const ProbeParams& P, Ctrl* ctrl) {
   }
 }
 
+// Fault injection (CDPROBE_OPT_DEBUG_DAMAGE_WRITE): the host put a damage code into the `writer` byte of a write
+// job (unused on write jobs).  The barrier leader that closes the job's phase applies it to the landing slot after
+// every local CTA has arrived and before anything is published, released or signalled: the loop-back's diagonal
+// verify starts as soon as the grid is released, a remote verify once this rank signals.  The writer's own (S, X)
+// stays that of the clean pattern.
+__device__ __noinline__ void damage_slot(const ProbeParams& P, const Job& job) {
+  uint8_t* pb = P.base_peer[job.peer];
+  if (pb == nullptr) return;
+  // TMA-path stores came through the async proxy: order them before this thread's generic accesses
+  fence_proxy_async_global();
+  uint64_t* w = reinterpret_cast<uint64_t*>(pb + P.land_off + (uint64_t)job.slot * P.bpp);
+  uint64_t* last = w + (P.bpp / 8 - 1);
+  switch (job.writer) {
+    case 1: st_relaxed_sys(w, ld_relaxed_sys(w) ^ 1ull); break;
+    case 2: st_relaxed_sys(last, ld_relaxed_sys(last) ^ (1ull << 63)); break;
+    case 3:
+      st_relaxed_sys(w, ld_relaxed_sys(w) + kGolden);
+      st_relaxed_sys(last, ld_relaxed_sys(last) - kGolden);
+      break;
+    case 4: {
+      const uint64_t w0 = ld_relaxed_sys(w), w1 = ld_relaxed_sys(w + 1);
+      st_relaxed_sys(w, w1);
+      st_relaxed_sys(w + 1, w0);
+      break;
+    }
+    default: break;
+  }
+  __threadfence_system();
+}
+
 __device__ __forceinline__ void signal_ranks(const ProbeParams& P, uint32_t mask, uint64_t target) {
   for (uint32_t j = 0; j < P.n_ranks; ++j) {
     if (j == P.rank || !((mask >> j) & 1u)) continue;
@@ -518,6 +548,13 @@ __device__ void barrier(const ProbeParams& P, Ctx& c, int b, uint32_t sync, uint
         *reinterpret_cast<volatile unsigned int*>(&ctrl->grid_arrive) = 0u;
         __threadfence();
         const uint64_t t_arr = gtimer();
+        if (b >= 1) {
+#pragma unroll
+          for (int jb = 0; jb < 2; ++jb) {
+            const Job& job = P.phase[b - 1].job[jb];
+            if (job.kind == kJobWrite && job.writer != 0) damage_slot(P, job);
+          }
+        }
         bool published = false, wrote_done = false;
         if (sync) {
           if (b >= 1) {

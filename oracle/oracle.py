@@ -150,6 +150,16 @@ def write_checksum(seed: int, src: int, dst: int, run_seq: int, n_words: int):
     return s.value, x.value
 
 
+def checksum(words):
+    """(S, X) of a numpy.uint64 array of words, by cdoracle_checksum (granules counted from words[0])."""
+    import numpy as np
+
+    w = np.ascontiguousarray(words, dtype=np.uint64)
+    s, x = C.c_uint64(), C.c_uint64()
+    lib().cdoracle_checksum(w.ctypes.data_as(C.POINTER(C.c_uint64)), w.size, C.byref(s), C.byref(x))
+    return s.value, x.value
+
+
 _GOLDEN = 0x9E3779B97F4A7C15
 _WRITE_TAG = 0x5752495445  # "WRITE"
 _M64 = (1 << 64) - 1
